@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("GWI_LIBRARY", os.path.join(_HERE, "libgwi.so"))  # override: tuning experiments only
+LIB_PATH = os.environ.get("GWI_LIBRARY", os.path.join(_HERE, "libgwi.so"))  # override: another build of the library, e.g. to compare two builds on the same GPU
 
 GWI_VERSION = 5  # include/gwi.h: GWI_VERSION (device-resident catalogs, device plan builder, plan timings in gwi_model_info)
 GWI_LIKE_HEADER = 8

@@ -30,7 +30,7 @@ unsigned stream_cta_smem_bytes(int nw, int ncol, int rows_total, int deep_entrie
 void launch_prologue_tables(const ModelDev* Md, const double* lam, int n_groups, int n_seg, bool two_pass, int nc, cudaStream_t st, int use_learned_shift);
 void launch_segmax_learn(const ModelDev* Md, int n_seg, int nc, cudaStream_t st);
 void launch_prologue_groups(const ModelDev* Md, const double* lam, int n_groups, int max_grid, int nc, cudaStream_t aux);
-void launch_reduce(const ModelDev* Md, int level, int n_tasks, int rec, int nc, int fan, cudaStream_t st);
+void launch_reduce(const ModelDev* Md, int level, int n_tasks, int rec, int nc, cudaStream_t st);
 void launch_segmax(const ModelDev* Md, int n_seg, int nc, cudaStream_t st);
 void launch_finish(const ModelDev* Md, int n_seg, int rec_doubles, int nc, cudaStream_t st);
 void launch_export(const ModelDev* Md, const gwi_outputs& out, cudaStream_t st);
@@ -751,11 +751,9 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
     }
     const char* g = std::getenv("GWI_GRAPH");
     m->use_graph = !(g && g[0] == '0') && !m->phase_timing;  // on by default (r02: +9 % e2e evals/s at config-2 size, bitwise-equal results)
-#if GWI_EXP_TRACK_MAX
     const char* sp = std::getenv("GWI_SPECULATIVE_SHIFT");
     m->spec_shift = H.two_pass && !(sp && sp[0] == '0');  // on by default (r02 call 37: cfg1 host call 308 -> 211 us, equal results)
     if (m->spec_shift) m->use_graph = false;  // the launch sequence differs from call to call
-#endif
   }
   m->stream_grid_x = std::max(1, std::min(p.grid_blocks, ((int)p.slice_begin.size() - 1 + p.warps_per_block - 1) / p.warps_per_block));
   m->max_grid_x = m->stream_grid_x;
@@ -772,7 +770,6 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
 
 // launches prologue .. finish for `nc` chains on `st` (lam_dev: [nc][P])
 static int run_eval(gwi_model* m, const double* lam_dev, int nc, cudaStream_t st, bool exact_shift = false) {
-  const Plan& p = m->plan;
   const ModelDev& H = m->host;
   phase_collect(m);
   phase_mark(m, 0, st);
@@ -802,7 +799,7 @@ static int run_eval(gwi_model* m, const double* lam_dev, int nc, cudaStream_t st
   }
   phase_mark(m, 2, st);
   const int n_levels = (int)m->level_tasks.size();
-  for (int l = 0; l + 1 < n_levels; ++l) launch_reduce(m->dev, l, m->level_tasks[l].second, H.rec_doubles, nc, l < (int)p.level_fan.size() ? p.level_fan[l] : 64, st);
+  for (int l = 0; l + 1 < n_levels; ++l) launch_reduce(m->dev, l, m->level_tasks[l].second, H.rec_doubles, nc, st);
   phase_mark(m, 3, st);
   cudaStreamWaitEvent(st, m->ev_join, 0);  // join
   // the last reduction level (one task per segment) is fused into finish_kernel

@@ -59,16 +59,13 @@ PdlLauncher<KArgs...> make_pdl_launcher(void (*k)(KArgs...), dim3 g, dim3 b, siz
 #define GWI_PDL_TRIGGER() asm volatile("griddepcontrol.launch_dependents;" ::: "memory")
 #endif
 
-// Speculative shift (GWI_EXP_TRACK_MAX, default 1; run-time switch GWI_SPECULATIVE_SHIFT=0 turns it off): models without an
+// Speculative shift (on by default; run-time switch GWI_SPECULATIVE_SHIFT=0 turns it off): models without an
 // a-priori bound of their log-weights (parametric terms, spline densities) need the exact per-segment maximum as the
 // log-sum-exp shift -- a max-only pass before the full pass.  Instead the full pass of the generic-term stream kernel also
 // records every chunk's max x, and the NEXT evaluation of gwi_loglike_host takes its shift from THIS evaluation's exact maxima;
 // an evaluation whose maxima moved by more than SPEC_SHIFT_TOL from the shift it used is flagged and repeated with the exact
 // maximum by the host call.  Measured on B200 (cfg1, profiles/r02_call37_speculative_shift.txt): host call 308 -> 211 us per
 // evaluation, results equal; the recording costs the spline-only kernels nothing (compiled into the PARAM variants only).
-#ifndef GWI_EXP_TRACK_MAX
-#define GWI_EXP_TRACK_MAX 1
-#endif
 
 namespace gwi {
 
@@ -147,7 +144,7 @@ struct ModelDev {
   double* seg_J1;     // [n_segments * P]
   double* seg_Jn;     // [n_segments * P]
   double* inj_raw;    // [3 + 2P] {shift, S1, S2, G1raw[P], G2raw[P]}
-  // speculative shift (GWI_EXP_TRACK_MAX): maxima learned from the last full pass; 1.0 where the shift used was too far off
+  // speculative shift: maxima learned from the last full pass; 1.0 where the shift used was too far off
   double* shift_next;  // [n_segments]
   double* spec_bad;    // [n_segments], zero unless a speculative evaluation has to be repeated
   // CTA-cooperative stream kernel (stream_cta.cuh): main warps per CTA (0 = the one-role kernel's geometry)

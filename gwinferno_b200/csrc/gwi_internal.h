@@ -19,12 +19,9 @@ constexpr int LANES = 32;
 constexpr int UNROLL = 2;           // samples per lane per load (16-byte vector loads)
 constexpr int CTA_STAGES = 4;       // stream_cta.cuh: staged 64-sample blocks per main warp (== CTA_NSTAGE)
 constexpr int CTA_WARPS_MAX = 12;   // stream_cta.cuh: main + deep warps per CTA (== CTA_MAX_WARPS)
-#ifndef GWI_DEEP_LANES
-#define GWI_DEEP_LANES 16
-#endif
-// copies of the deep accumulators per warp: 16 = lanes l and l+16 share a slot (two update phases,
-// half the shared memory), 32 = fully lane-private (one phase)
-constexpr int DEEP_LANES = GWI_DEEP_LANES;
+// copies of the deep accumulators per warp: lanes l and l+16 share a slot (two update phases, half the
+// shared memory of fully lane-private copies)
+constexpr int DEEP_LANES = 16;
 
 // ---- packed spline word: the fp64 value w = u - 1/2 (u in [0,1): offset inside the polynomial piece)
 // with its 6 least significant mantissa bits replaced by the piece index J.  The kernels use the word
@@ -145,7 +142,6 @@ struct Plan {
   // tasks of the segments that still have more than one fan-in of inputs (a 10 000-sample event goes straight from its
   // few records to the last level instead of being copied through every level)
   std::vector<std::vector<ReduceTask>> levels;
-  std::vector<int> level_fan;  // fan-in (64 / 128 / 256) of every level but the last
   // launch geometry (fixed at plan time: the chunk -> warp assignment depends on it)
   int grid_blocks = 0, warps_per_block = 0;
   int chunk_steps = 0;

@@ -20,14 +20,9 @@
 
 #include "dev_structs.h"
 
-// GWI_EXP_STAGE_DESC (on since round 2; =0 restores direct reads): the small kernels read dozens of ModelDev fields,
-// each a dependent global load (the cold prologue takes 33 us under ncu, mostly load latency).  With
-// the switch a block first copies its chain's descriptor (~3 KB) into shared memory with coalesced
-// 8-byte loads and works from that copy.
-#ifndef GWI_EXP_STAGE_DESC
-#define GWI_EXP_STAGE_DESC 1
-#endif
-#if GWI_EXP_STAGE_DESC
+// The small kernels read dozens of ModelDev fields, each a dependent global load if read in place (the cold
+// prologue took 33 us under ncu, mostly load latency).  So a block first copies its chain's descriptor (~3 KB)
+// into shared memory with coalesced 8-byte loads and works from that copy.
 #define GWI_STAGED_DESC(M, src)                                                                              \
   __shared__ __align__(16) unsigned long long gwi_desc_stage[(sizeof(ModelDev) + 7) / 8];                    \
   {                                                                                                          \
@@ -36,9 +31,6 @@
     __syncthreads();                                                                                         \
   }                                                                                                          \
   const ModelDev& M = *reinterpret_cast<const ModelDev*>(gwi_desc_stage)
-#else
-#define GWI_STAGED_DESC(M, src) const ModelDev& M = (src)
-#endif
 
 namespace gwi {
 
@@ -467,12 +459,12 @@ __device__ __forceinline__ double reduce_element(const ModelDev& M, const Reduce
   return ((a[0] + a[1]) + (a[2] + a[3])) + ((a[4] + a[5]) + (a[6] + a[7]));
 }
 
-// One block = one task x 32 record elements; the 8 warps split the task's <= 64 / 128 / 256 inputs (warp g takes inputs g, g+8, ...:
-// at most K = 8 / 16 / 32 independent loads per thread, ONE memory round trip) and the partial sums are combined through shared memory in
+// One block = one task x 32 record elements; the 8 warps split the task's <= 64 inputs (warp g takes inputs g, g+8, ...:
+// at most K = 8 independent loads per thread, ONE memory round trip) and the partial sums are combined through shared memory in
 // the same fixed order as reduce_element's.  (A thread per element walking all 64 inputs needed 8 dependent rounds: ~20 us per
 // level whatever the number of tasks.)
-template <int K>  // K = fan-in / 8 loads per thread
 __global__ void __launch_bounds__(256) reduce_kernel(const ModelDev* __restrict__ Mp, int level) {
+  constexpr int K = 8;  // loads per thread: fan-in 64 / 8 warps
   GWI_PDL_TRIGGER();
   const ModelDev& M = Mp[blockIdx.z];  // blockIdx.z = chain
   const ReduceTask T = M.level_tasks[level][blockIdx.x];  // (static data: read before the dependency wait)
@@ -517,7 +509,7 @@ __global__ void __launch_bounds__(256) segmax_kernel(const ModelDev* __restrict_
   if (threadIdx.x == 0) M.shift[s] = (mx > -INFINITY && mx < INFINITY) ? mx : 0.0;
 }
 
-// after a full pass that recorded the chunk maxima (GWI_EXP_TRACK_MAX): learn the next evaluation's shift and
+// after a full pass that recorded the chunk maxima (speculative shift): learn the next evaluation's shift and
 // flag the segments whose maximum is too far from the shift this evaluation used
 __global__ void __launch_bounds__(256) segmax_learn_kernel(const ModelDev* __restrict__ Mp) {
   const ModelDev& M = Mp[blockIdx.y];
@@ -551,9 +543,7 @@ __device__ void finish_segment(const ModelDev& M, int s, const double* rec) {
   double K = M.Ksum[0];
   for (int g = 0; g < M.n_groups; ++g) K -= M.logZ[g];
   bool ok = (S1 > 0.0) && (S1 < INFINITY) && (S2 > 0.0) && (S2 < INFINITY);
-#if GWI_EXP_TRACK_MAX
   ok = ok && M.spec_bad[s] == 0.0;  // the learned shift was too far from this evaluation's maximum
-#endif
   const double N = M.total_inj;
   const double den_inj = S2 - S1 * S1 / N;
   if (threadIdx.x == 0) {
@@ -966,11 +956,8 @@ void launch_segmax_learn(const ModelDev* Md, int n_seg, int nc, cudaStream_t st)
 void launch_prologue_groups(const ModelDev* Md, const double* lam, int n_groups, int max_grid, int nc, cudaStream_t aux) {
   if (n_groups > 0) GWI_LAUNCH(prologue_kernel, dim3(n_groups, nc), 256, (size_t)max_grid * sizeof(double), aux)(Md, lam, 0, 0);
 }
-void launch_reduce(const ModelDev* Md, int level, int n_tasks, int rec, int nc, int fan, cudaStream_t st) {
-  dim3 grid(n_tasks, (rec + 31) / 32, nc);
-  if (fan <= 64) GWI_LAUNCH_PDL(reduce_kernel<8>, grid, 256, 0, st)(Md, level);
-  else if (fan <= 128) GWI_LAUNCH_PDL(reduce_kernel<16>, grid, 256, 0, st)(Md, level);
-  else GWI_LAUNCH_PDL(reduce_kernel<32>, grid, 256, 0, st)(Md, level);
+void launch_reduce(const ModelDev* Md, int level, int n_tasks, int rec, int nc, cudaStream_t st) {
+  GWI_LAUNCH_PDL(reduce_kernel, dim3(n_tasks, (rec + 31) / 32, nc), 256, 0, st)(Md, level);
 }
 void launch_segmax(const ModelDev* Md, int n_seg, int nc, cudaStream_t st) { GWI_LAUNCH(segmax_kernel, dim3(n_seg, nc), 256, 0, st)(Md); }
 void launch_finish(const ModelDev* Md, int n_seg, int rec_doubles, int nc, cudaStream_t st) {

@@ -886,7 +886,6 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
       const int64_t fixed = 3 * 8 * CTA_STAGES * CTA_WARPS_MAX + 16 + (int64_t)plan.rows_total * 32 + 256 + (int64_t)rows_deep * (1024 + 256);
       int nw = (int)((226 * 1024 - fixed) / (CTA_STAGES * stage_bytes));
       nw = std::min(nw, CTA_WARPS_MAX - plan.n_deep);
-      if (const char* e = std::getenv("GWI_TUNE_CTA_WARPS")) nw = std::min(nw, std::max(1, std::atoi(e)));
       if (nw >= 2) {
         plan.cta_mode = true;
         plan.cta_main_warps = nw;
@@ -895,13 +894,12 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
   }
   const int LW = plan.cta_mode ? plan.cta_main_warps : 1;  // warps that share a chunk
   const int LPC = LANES * LW;                              // lane runs per chunk
-  // GWI_TUNE_BATCH_HINT=n (tuning experiment, default 1): the model will be evaluated for ~n chains per
-  // launch (gwi_loglike_batch), so the machine is filled by chains and ONE chain only needs W/n warps:
+  // gwi_model_desc.batch_hint = n (default 1): the model will be evaluated for ~n chains per launch
+  // (gwi_loglike_batch), so the machine is filled by chains and ONE chain only needs W/n warps:
   // slices get n times longer (up to the cap), i.e. fewer record flushes and longer piece-sorted lane
   // runs.  The emulator's path statistics for the config-2 catalog: 2 701 chunks of 8 steps and 88 % of
   // the warp iterations with lanes on the piece-change path at n = 1.
-  int batch_hint = std::max(1, (int)desc.batch_hint);  // gwi_model_desc.batch_hint: chains per gwi_loglike_batch call
-  if (const char* e = std::getenv("GWI_TUNE_BATCH_HINT")) batch_hint = std::max(1, std::atoi(e));
+  const int batch_hint = std::max(1, (int)desc.batch_hint);
   plan.batch_hint = batch_hint;
   const int W = plan.cta_mode ? std::max(1, plan.grid_blocks / batch_hint) : std::max(plan.warps_per_block, plan.grid_blocks * plan.warps_per_block / batch_hint);
   // Balanced slicing: the piece-sorted sample stream of all segments (the events first, then the
@@ -922,9 +920,8 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
   const int64_t per_warp = (total_steps + W - 1) / W;
   // slices per warp the one-role kernel aims for: 4 on long catalogs, 2 where a warp only has a few hundred steps (an 8-way cfg3
   // shard, 330 steps per warp: 4308 instead of 5764 chunks, step 0.304 -> 0.296 ms; cfg3 itself 1.600 vs 1.624 ms the other way:
-  // profiles/r02_call29_slices.txt).  GWI_TUNE_SLICES_PER_WARP overrides (tuning experiments).
-  int64_t spw = per_warp < 512 ? 2 : 4;
-  if (const char* e = std::getenv("GWI_TUNE_SLICES_PER_WARP")) spw = std::max(1, std::atoi(e));
+  // profiles/r02_call29_slices.txt).
+  const int64_t spw = per_warp < 512 ? 2 : 4;
   int64_t L = roundQ(std::max<int64_t>(per_warp < 64 ? 32 : 64, std::min<int64_t>(768, per_warp / spw)));
   L = std::max<int64_t>(L, 8 * Q);
   bool fixed_L = false;  // one slice per CTA: no guided shrink
@@ -932,17 +929,14 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
     // a slice is L steps of ALL main warps of a CTA: >= ~4 slices per CTA for the dynamic balance, but never
     // fewer slices than CTAs on a small catalog
     // r02 sweeps (B200, ms/step at div = 1 / 2 / 3 / 4): 8-way cfg3 shard 0.390 / 0.327 / 0.325 / 0.331, cfg5 - / 0.531 / 0.539 / 0.539
-    int64_t div = 2;
-    if (const char* e = std::getenv("GWI_TUNE_SLICE_DIV")) div = std::max(1, std::atoi(e));
+    const int64_t div = 2;
     L = roundQ(std::min<int64_t>(768, std::max<int64_t>(16, per_warp / div)));
     if (L > per_warp) L = roundQ(std::max<int64_t>(Q, per_warp));
     // Small catalogs (a few blocks per warp: the kernel is latency, not throughput): every slice costs a counter round trip,
     // a pipeline fill and a record flush, so give every CTA exactly ONE slice -- the shortest L whose slice count still fits
     // the grid (cfg2, 70 events of 18 steps + 2232 injection steps on 148 CTAs: L = 30 -> 145 slices / 145 chunks instead of
-    // L = 16 -> 280 chunks, where every event was cut into a 16-step and a 2-step chunk).  GWI_TUNE_ONE_SLICE=0 disables.
-    bool one_slice = per_warp < 64;
-    if (const char* e = std::getenv("GWI_TUNE_ONE_SLICE")) one_slice = one_slice && e[0] != '0';
-    if (one_slice) {
+    // L = 16 -> 280 chunks, where every event was cut into a 16-step and a 2-step chunk).
+    if (per_warp < 64) {
       auto n_slices_for = [&](int64_t Lt) {
         int64_t slices = 1, fill_t = 0;
         for (int si = 0; si < n_seg; ++si) {
@@ -979,23 +973,16 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
   plan.slice_begin.clear();
   plan.slice_begin.push_back(0);
   // Guided scheduling: the warps pull slices in order, so the slices shrink towards the end of
-  // the stream (guided self-scheduling: slice = remaining work / 2W, clamped to [8, L]) to keep
+  // the stream (guided self-scheduling: slice = remaining work / W, clamped to [L_MIN, L]) to keep
   // the tail short.
   const int64_t L_full = L;
   // one warp step takes ~2500 cycles of latency (8 resident warps/SM), so a 32-step final slice is a
   // 40 us tail; 8-step slices at the very end cut it to ~10 us for ~2W extra record flushes
-  // tuning experiments only (defaults = the measured choice): GWI_TUNE_LMIN, GWI_TUNE_GUIDED_DIV
-  auto env_int = [](const char* name, int64_t dflt, int64_t lo, int64_t hi) {
-    const char* v = std::getenv(name);
-    if (!v || !*v) return dflt;
-    const long long x = std::atoll(v);
-    return (int64_t)std::min<long long>(hi, std::max<long long>(lo, x));
-  };
   // r02 measurements (B200): DIV 1 / LMIN 32 instead of 2 / 8 cut the chunks of an 8-way cfg3 shard from 10 044 to 5 764 and its
   // stream kernel from 0.427 to 0.372 ms, the full catalog from 15 167 to 8 477 chunks and 1.807 to 1.752 ms (fewer record
   // flushes and records to reduce; the tail stays short because the final slices are still small)
-  const int64_t L_MIN = fixed_L ? L : roundQ(env_int("GWI_TUNE_LMIN", 32, Q, 1024));
-  const int64_t GUIDED_DIV = env_int("GWI_TUNE_GUIDED_DIV", 1, 1, 16);  // slice = remaining / (DIV * W)
+  const int64_t L_MIN = fixed_L ? L : roundQ(32);
+  const int64_t GUIDED_DIV = 1;  // slice = remaining / (DIV * W)
   int64_t done_steps = 0;
   int64_t pos = 0, fill = 0;
   for (int si = 0; si < n_seg; ++si) {
@@ -1205,24 +1192,17 @@ void plan_tree(Plan& plan) {
     }
     for (int s = 0; s < n_seg; ++s) first[s] = plan.segments[s].first_chunk * RPC;  // chunks (hence records) of a segment are consecutive
     // reduction tree, fan-in 64: per segment, levels are added only while it has more than LAST = 64 inputs (what
-    // finish_kernel sums itself).  A larger fan-in (128 / 256: GWI_TUNE_REDUCE_FAN, reduce_kernel<16 / 32>) would bring cfg3's
+    // finish_kernel sums itself).  A larger fan-in (128 / 256) would bring cfg3's
     // 8477 records down in ONE level instead of two, i.e. one dependent launch less -- measured SLOWER on B200
     // (profiles/r02_call31_reduce_fan.txt: everything-but-the-stream-kernel per evaluation 76.7 us with two levels of 64 against
     // 99-108 us with one level of 128 / 256 on cfg3, 69.6 against 78-83 us on an 8-way shard, 76 against 89-96 us on cfg5:
     // finish_kernel's injection block then sums 34-67 inputs itself, which costs more than the extra launch).  64 it stays.
-    constexpr int LAST = 64;
-    plan.level_fan.clear();
+    constexpr int LAST = 64, FAN = 64;  // FAN: reduce_kernel's fixed fan-in
     std::vector<int> src(n_seg, -1);  // where the segment's current inputs are (-1 = level-0 records)
     for (;;) {
       int max_cnt = 0;
       for (int s = 0; s < n_seg; ++s) max_cnt = std::max(max_cnt, cnt[s]);
       if (max_cnt <= LAST) break;
-      int FAN = 64;
-      if (const char* e = std::getenv("GWI_TUNE_REDUCE_FAN")) {  // tuning experiments: force 64 / 128 / 256
-        const int v = std::atoi(e);
-        if (v == 64 || v == 128 || v == 256) FAN = v;
-      }
-      plan.level_fan.push_back(FAN);
       const int lvl = (int)plan.levels.size();
       std::vector<ReduceTask> tasks;
       for (int s = 0; s < n_seg; ++s) {

@@ -466,9 +466,6 @@ static void install_debug_handler() {
 
 extern "C" {
 
-// counters of -DGWI_EMU_STATS builds (see csrc/stream.cuh); read and cleared from Python through ctypes
-unsigned long long gwi_emu_stats[16] = {0};
-
 int gwi_emu_marker(void) {
   install_debug_handler();
   return 1;

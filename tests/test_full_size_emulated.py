@@ -23,7 +23,7 @@ from tests import emu
 def _emulated_b200():
     old = os.environ.get("GWI_EMU_SMS")
     os.environ["GWI_EMU_SMS"] = "148"
-    variant = os.environ.get("GWI_EMU_VARIANT", "")  # an experiment build made by hand (tests/emu/Makefile VARIANT=)
+    variant = os.environ.get("GWI_EMU_VARIANT", "")  # a variant build made by hand (tests/emu/Makefile VARIANT=, e.g. ASan)
     try:
         if not variant:
             emu.build()

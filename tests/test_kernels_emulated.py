@@ -32,7 +32,7 @@ del _name
 
 @pytest.fixture(scope="module", autouse=True)
 def _emulated_device():
-    variant = os.environ.get("GWI_EMU_VARIANT", "")  # an experiment build (tests/emu/Makefile VARIANT=), built by hand
+    variant = os.environ.get("GWI_EMU_VARIANT", "")  # a variant build (tests/emu/Makefile VARIANT=, e.g. ASan), built by hand
     try:
         if not variant:
             emu.build()

@@ -1,8 +1,8 @@
 """CPU: randomised differential test of the kernel sources (on the host warp emulator, tests/emu) against
 the NumPy oracle: random catalog sizes (down to one sample per event), spline counts, coefficient
 scales, deep-dim splits, chunk lengths, N_eff gradients on / off and both epilogues.  Values to 1e-10,
-Jacobians to 1e-8 (observed over 450 configurations: 1.4e-14 / 8.5e-14).  GWI_EMU_VARIANT selects an
-experiment build, GWI_FUZZ_CASES / GWI_FUZZ_SEED widen the search."""
+Jacobians to 1e-8 (observed over 450 configurations: 1.4e-14 / 8.5e-14).  GWI_EMU_VARIANT selects a
+variant build (e.g. ASan), GWI_FUZZ_CASES / GWI_FUZZ_SEED widen the search."""
 
 import os
 

@@ -61,8 +61,3 @@ for w in "cfg3" "cfg3 --emulate-world 8" "cfg2 --steps 300 --warmup 20" "cfg5"; 
 done
 cat "$OUT/${TAG}_phases.txt"
 ls -la "$OUT" | grep "${TAG}" | tail -30
-# slice-length sweep of the CTA-cooperative kernel on the shard (tuning evidence)
-for d in 1 2 3; do
-  GWI_TUNE_SLICE_DIV=$d python bench.py --workload cfg3 --emulate-world 8 --steps 100 --no-cpu-baseline 2>/dev/null | python -c "
-import json,sys; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print('shard8 slice_div=$d', round(d['ms_per_step'],4), 'ms/step kernel', round(d['roofline']['kernel_ms'],4), 'chunks', d['plan']['n_chunks'])" | tee -a "$OUT/${TAG}_shard8_slice_div.txt"
-done
