@@ -97,7 +97,8 @@ typedef struct {
   int32_t col[2];     /* catalog column indices, -1 if unused */
   int32_t slot[6];    /* offsets into Lambda, -1 if unused; SPLINE: slot[0] = first coefficient */
   double cst[4];      /* constants, see gwi_term_kind */
-  int32_t n_splines;  /* SPLINE: number of basis functions (>= 4, <= 256) */
+  int32_t n_splines;  /* SPLINE: number of basis functions, >= 4; at most 64 with the default knots, and with an
+                         explicit knot vector at most 61 polynomial pieces inside [xi_lo, xi_hi] */
   int32_t norm_group; /* index into groups[], -1 = term has no grid normaliser */
   double x_lo, x_hi;   /* SPLINE: support in col0 units (the model mask) */
   double xi_lo, xi_hi; /* SPLINE: support in spline-coordinate units (= log of the above if logx) */
