@@ -16,6 +16,7 @@
 
 #include "dev_structs.h"
 #include "plan_sample.h"
+#include "smem_layout.h"
 
 namespace gwi {
 
@@ -26,7 +27,6 @@ typedef void (*stream_fn)(const ModelDev*);
 stream_fn pick_stream_kernel(int ns, int ndeep, int nlin, bool g2, bool param, bool maxonly);
 stream_fn pick_stream_cta_kernel(int ns, int ndeep, int nlin);  // CTA-cooperative kernel (stream_cta.cuh)
 stream_fn pick_stream_cta_max_kernel();
-unsigned stream_cta_smem_bytes(int nw, int ncol, int rows_total, int deep_entries);
 void launch_prologue_tables(const ModelDev* Md, const double* lam, int n_groups, int n_seg, bool two_pass, int nc, cudaStream_t st, int use_learned_shift);
 void launch_segmax_learn(const ModelDev* Md, int n_seg, int nc, cudaStream_t st);
 void launch_prologue_groups(const ModelDev* Md, const double* lam, int n_groups, int max_grid, int nc, cudaStream_t aux);
@@ -560,7 +560,7 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
   H.two_pass = 0;
   H.liny_mask = 0;
   const int mom = p.g2 ? 2 : 1;
-  int deep_entries = 0;
+  int deep_rows = 0;
   for (int d = 0; d < NS; ++d) {
     const SplineDim& D = p.dims[d];
     const gwi_term& t = desc->terms[D.term];
@@ -570,8 +570,8 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
     X.slot = D.slot;
     X.n_splines = D.n_splines;
     X.deep = D.deep;
-    X.deep_off = D.deep ? deep_entries : 0;
-    if (D.deep) deep_entries += D.rows * 2 * mom;  // double2 entries
+    X.deep_off = D.deep ? deep_rows * 2 * mom : 0;  // first double2 accumulator (smem_layout.h): (row, moment set, pair)
+    if (D.deep) deep_rows += D.rows;
     X.norm_group = D.norm_group;
     X.grid_off = D.grid_off;
     X.grid_aux = D.grid_aux;
@@ -587,7 +587,7 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
     X.xi_lo = t.xi_lo;
     X.inv_dxi = (double)(D.rows - 1) / (t.xi_hi - t.xi_lo);
   }
-  H.deep_entries = deep_entries;
+  H.deep_rows = deep_rows;
   if (p.cta_mode) {
     // what a main warp of the CTA-cooperative kernel writes of its record: {S1, S2}, the linear-term slots and the rows of
     // the leading dims (the dims are in sort-key order, the deep ones last)
@@ -712,30 +712,24 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
     gwi_model_destroy(m);
     return GWI_ERR_UNSUPPORTED;
   }
-  const size_t per_warp = (size_t)p.rows_total * 4 * mom + (size_t)deep_entries * 2 * DEEP_LANES + (size_t)p.n_gslots * 32 * (1 + mom);  // deep: double2 x DEEP_LANES copies
-  const size_t fixed = (size_t)p.rows_total * 4 + (size_t)(deep_entries / (2 * mom)) * 32 + (size_t)H.n_kops * KC_STRIDE + (size_t)H.n_kops * (sizeof(KopDev) / 8);
-  static_assert(sizeof(KopDev) % 16 == 0, "KopDev copies must keep the shared layout 16-byte aligned");
-  int wpb = p.warps_per_block;
-  while (wpb > 1 && (fixed + per_warp * wpb) * 8 > (size_t)prop.sharedMemPerBlockOptin) --wpb;
-  if (wpb != p.warps_per_block) {
-    set_error("internal: plan geometry does not fit the device's shared memory");
-    gwi_model_destroy(m);
-    return GWI_ERR_UNSUPPORTED;
-  }
-  m->smem_full = (fixed + per_warp * wpb) * 8;
-  m->smem_max = m->smem_full;
-  m->stream_block = wpb * 32;
-  m->max_block = wpb * 32;
+  bool aligned = true;
   if (m->cta) {
-    m->smem_full = stream_cta_smem_bytes(p.cta_main_warps, p.n_columns, p.rows_total, deep_entries);
+    const CtaLayout L = cta_layout(p.cta_main_warps, p.n_columns, p.rows_total, deep_rows);
+    aligned = L.aligned16();
+    m->smem_full = L.total;
     m->smem_max = 0;
     m->stream_block = (p.cta_main_warps + p.n_deep) * 32;
     m->max_block = 256;
-    if (m->smem_full == 0 || m->smem_full > (size_t)prop.sharedMemPerBlockOptin) {
-      set_error("internal: CTA-kernel geometry does not fit the device's shared memory");
-      gwi_model_destroy(m);
-      return GWI_ERR_UNSUPPORTED;
-    }
+  } else {
+    m->smem_full = one_role_smem_bytes(p.rows_total, deep_rows, mom, H.n_kops, p.n_gslots, p.warps_per_block);
+    m->smem_max = m->smem_full;
+    m->stream_block = p.warps_per_block * 32;
+    m->max_block = p.warps_per_block * 32;
+  }
+  if (!aligned || m->smem_full > (size_t)prop.sharedMemPerBlockOptin) {
+    set_error("internal: plan geometry does not fit the device's shared memory");
+    gwi_model_destroy(m);
+    return GWI_ERR_UNSUPPORTED;
   }
   if (cudaFuncSetAttribute((const void*)m->k_full, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_full) != cudaSuccess ||
       cudaFuncSetAttribute((const void*)m->k_max, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->smem_max) != cudaSuccess) {

@@ -110,7 +110,7 @@ struct GroupDev {
 // descriptor array with their chain coordinate of the grid
 struct ModelDev {
   int32_t n_params, n_dims, n_deep, n_kops, n_gslots, n_sops, n_groups, n_segments;
-  int32_t rows_total, rec_doubles, n_columns, col_static, g2, two_pass, n_chunks, deep_entries;
+  int32_t rows_total, rec_doubles, n_columns, col_static, g2, two_pass, n_chunks, deep_rows;  // deep_rows: table rows of the deep dims
   int32_t n_lin_fast, n_slices;  // leading LIN kops handled in registers by the stream kernel
   int64_t n_padded;
   double total_inj;

@@ -7,6 +7,17 @@
 
 #include "gwi.h"
 
+// host + device functions (the plan builders' per-sample arithmetic, the shared-memory layouts); plain functions in
+// the host warp emulator's g++ build.  GWI_HD_INLINE: inlined before the caller is optimised, so that the caller compiles
+// as if the body were written out in it.
+#if defined(__CUDACC__) && !defined(GWI_HOST_EMULATION)
+#define GWI_HD __host__ __device__
+#define GWI_HD_INLINE __host__ __device__ __forceinline__
+#else
+#define GWI_HD
+#define GWI_HD_INLINE inline
+#endif
+
 namespace gwi {
 
 constexpr int MAX_SPLINE_DIMS = 8;  // spline dimensions per model
@@ -17,8 +28,6 @@ constexpr int MAX_SOPS = 16;        // scalar (sample-independent) normaliser op
 constexpr int KC_STRIDE = 12;       // doubles of per-eval constants per kop
 constexpr int LANES = 32;
 constexpr int UNROLL = 2;           // samples per lane per load (16-byte vector loads)
-constexpr int CTA_STAGES = 4;       // stream_cta.cuh: staged 64-sample blocks per main warp (== CTA_NSTAGE)
-constexpr int CTA_WARPS_MAX = 12;   // stream_cta.cuh: main + deep warps per CTA (== CTA_MAX_WARPS)
 // copies of the deep accumulators per warp: lanes l and l+16 share a slot (two update phases, half the
 // shared memory of fully lane-private copies)
 constexpr int DEEP_LANES = 16;

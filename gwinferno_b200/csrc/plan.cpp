@@ -24,6 +24,7 @@
 
 #include "gwi_internal.h"
 #include "plan_sample.h"
+#include "smem_layout.h"
 
 namespace gwi {
 
@@ -793,7 +794,6 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
   const bool timing = tm.on;
   const int NS = (int)plan.dims.size();
   const int n_seg = (int)plan.segments.size();
-  const std::vector<Feat>& kop_feats = in.kop_feats;
   chunk_r0.clear();
   chunk_nc.clear();
   bool want_cta = false;  // the CTA-cooperative stream kernel is the better one for this plan (decided below)
@@ -864,32 +864,26 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
     for (int d = 0; d < NS; ++d) plan.dims[d].deep = d >= NS - nd;
   }
   // ---- launch geometry + chunking -----------------------------------------------------------
-  // shared memory per warp: shallow accumulators + deep lane-private arrays + generic slots
+  // the most warps whose exact shared-memory layout (smem_layout.h) fits SMEM_BUDGET, 225 of the 227 KB an sm_100 CTA
+  // may use.  The warp counts fix the chunking, hence the summation order: another budget moves results in the last bits.
+  constexpr unsigned SMEM_BUDGET = 225 * 1024;
   const int mom = plan.g2 ? 2 : 1;
   int rows_deep = 0;
   for (int d = 0; d < NS; ++d)
     if (plan.dims[d].deep) rows_deep += plan.dims[d].rows;
-  const int64_t warp_bytes = (int64_t)plan.rows_total * 4 * mom * 8 + (int64_t)rows_deep * 4 * mom * DEEP_LANES * 8 +
-                             (int64_t)plan.n_gslots * (1 + mom) * LANES * 8;
-  const int64_t cta_fixed = (int64_t)plan.rows_total * 4 * 8 + (int64_t)rows_deep * 256 + (int64_t)plan.kops.size() * (KC_STRIDE * 8 + 80) + 1024;
-  int wpb = (int)((226 * 1024 - cta_fixed) / std::max<int64_t>(1, warp_bytes));  // 227 KB per CTA on sm_100; api.cu re-checks with the exact layout
-  wpb = std::max(1, std::min(wpb, 8));
+  int wpb = 8;
+  while (wpb > 1 && one_role_smem_bytes(plan.rows_total, rows_deep, mom, (int)plan.kops.size(), plan.n_gslots, wpb) > SMEM_BUDGET) --wpb;
   plan.warps_per_block = wpb;
   plan.grid_blocks = std::max(1, sm_count);
   // CTA-cooperative geometry (stream_cta.cuh) for spline models with at most 2 linear terms and no N_eff
   // gradient: main warps stage their blocks with bulk copies, one dedicated warp per deep dim accumulates
   // that dim's moments for the whole CTA.  GWI_CTA_KERNEL=0 keeps the one-role kernel (tuning / bisection).
-  {
-    const bool ok = want_cta && plan.n_deep >= 1;
-    if (ok) {
-      const int64_t stage_bytes = (int64_t)(NS + (int)kop_feats.size() + 1) * 512 + 512;
-      const int64_t fixed = 3 * 8 * CTA_STAGES * CTA_WARPS_MAX + 16 + (int64_t)plan.rows_total * 32 + 256 + (int64_t)rows_deep * (1024 + 256);
-      int nw = (int)((226 * 1024 - fixed) / (CTA_STAGES * stage_bytes));
-      nw = std::min(nw, CTA_WARPS_MAX - plan.n_deep);
-      if (nw >= 2) {
-        plan.cta_mode = true;
-        plan.cta_main_warps = nw;
-      }
+  if (want_cta && plan.n_deep >= 1) {
+    int nw = CTA_MAX_WARPS - plan.n_deep;
+    while (nw >= 2 && cta_layout(nw, plan.n_columns, plan.rows_total, rows_deep).total > SMEM_BUDGET) --nw;
+    if (nw >= 2) {
+      plan.cta_mode = true;
+      plan.cta_main_warps = nw;
     }
   }
   const int LW = plan.cta_mode ? plan.cta_main_warps : 1;  // warps that share a chunk

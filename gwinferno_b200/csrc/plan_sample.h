@@ -11,12 +11,6 @@
 
 #include "gwi_internal.h"
 
-#if defined(__CUDACC__) && !defined(GWI_HOST_EMULATION)
-#define GWI_HD __host__ __device__
-#else
-#define GWI_HD
-#endif
-
 namespace gwi {
 
 GWI_HD inline double plan_nan() {

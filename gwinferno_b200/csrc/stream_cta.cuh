@@ -27,27 +27,6 @@
 
 namespace gwi {
 
-constexpr int CTA_NSTAGE = 4;
-constexpr int CTA_MAX_WARPS = 12;  // main + deep warps (launch bound 384 threads => 168 registers; 13 warps make ptxas fall back to 128 + spills)
-
-// shared-memory layout of the CTA kernel (bytes from the start of the dynamic shared memory)
-struct CtaLayout {
-  unsigned bars, ctl, tables, dtab, stages, stage_bytes, blk_bytes, deep, total;
-};
-__host__ __device__ inline CtaLayout cta_layout(int nw, int ncol, int rows_total, int deep_entries) {
-  CtaLayout L;
-  L.bars = 0;  // mbarriers: full[nw][NSTAGE] (one per staged block) | ready[NSTAGE] (count nw) | free[NSTAGE] (count n_deep)
-  L.ctl = (L.bars + ((unsigned)nw + 2u) * CTA_NSTAGE * 8u + 15u) & ~15u;  // 16 B: slice id broadcast (16-byte aligned: the tables follow)
-  L.tables = L.ctl + 16u;
-  L.blk_bytes = (unsigned)ncol * 512u;
-  L.stage_bytes = L.blk_bytes + 512u;                       // + the 64 weights p of the block
-  L.dtab = L.tables + (unsigned)rows_total * 32u;  // deep-dim half-rows replicated 8x: [h][r][lane & 7] double2 (conflict-free LDS.128)
-  L.stages = (L.dtab + (unsigned)(deep_entries / 2) * 256u + 127u) & ~127u;
-  L.deep = L.stages + (unsigned)nw * CTA_NSTAGE * L.stage_bytes;
-  L.total = L.deep + (unsigned)deep_entries * 32u * 16u;    // double2 [entry][lane]
-  return L;
-}
-
 // ---- mbarrier + bulk-copy primitives ------------------------------------------------------------
 #ifdef GWI_HOST_EMULATION
 #include <cstdio>
@@ -166,7 +145,7 @@ __global__ void __launch_bounds__(CTA_MAX_WARPS * 32, 1) stream_cta_kernel(const
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int NW = M.cta_main_warps;
   const int ncol = M.n_columns, rows_total = M.rows_total, n_gs = M.n_gslots;
-  const CtaLayout L = cta_layout(NW, ncol, rows_total, M.deep_entries);
+  const CtaLayout L = cta_layout(NW, ncol, rows_total, M.deep_rows);  // smem_layout.h
   double* const tables = reinterpret_cast<double*>(smb + L.tables);
   volatile int* const ctl = reinterpret_cast<volatile int*>(smb + L.ctl);
   // Synchronisation (all mbarriers, phases = uses of a stage):
@@ -184,7 +163,7 @@ __global__ void __launch_bounds__(CTA_MAX_WARPS * 32, 1) stream_cta_kernel(const
 
   {
     double2* dz = reinterpret_cast<double2*>(smb + L.deep);
-    for (int i = threadIdx.x; i < M.deep_entries * 32; i += blockDim.x) dz[i] = make_double2(0.0, 0.0);
+    for (int i = threadIdx.x; i < M.deep_rows * 64; i += blockDim.x) dz[i] = make_double2(0.0, 0.0);  // [row][moment pair][32 lanes]
   }
   if (threadIdx.x == 0) {
     for (int s = 0; s < CTA_NSTAGE; ++s) {

@@ -49,11 +49,4 @@ stream_fn pick_stream_cta_kernel(int ns, int ndeep, int nlin) {
   return nullptr;
 }
 stream_fn pick_stream_cta_max_kernel() { return (stream_fn)stream_cta_max_kernel<0>; }
-unsigned stream_cta_smem_bytes(int nw, int ncol, int rows_total, int deep_entries) {
-  const CtaLayout L = cta_layout(nw, ncol, rows_total, deep_entries);
-  // 16-byte vector accesses everywhere (tables, staged blocks, accumulators): 0 = a layout bug, refused by the caller
-  if ((L.ctl | L.tables | L.stages | L.stage_bytes | L.blk_bytes | L.deep) & 15u) return 0u;
-  return L.total;
-}
 }  // namespace gwi
-static_assert(gwi::CTA_STAGES == gwi::CTA_NSTAGE && gwi::CTA_WARPS_MAX == gwi::CTA_MAX_WARPS, "plan.cpp sizes the CTA geometry with the kernel's constants");
