@@ -617,6 +617,10 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
   for (int q = 0; q < H.n_sops; ++q) {
     const Sop& S = p.sops[q];
     H.sops[q] = SopDev{S.kind, S.slot[0], S.slot[1], 0, S.cst[0], S.cst[1]};
+    // A Beta term's two linear features, log x and log(s - x), peak at opposite ends of its support, so the sum of
+    // their separate maxima overshoots the largest weight by up to ~(a + b - 2) log 2: ~690 at a = b = 500, where every
+    // weight more than e^-16 below the largest one fell under the stream kernel's underflow cut.  Exact max first.
+    if (S.kind == SOP_BETA_NORM) H.two_pass = 1;
   }
   m->max_grid = 1;
   std::vector<GroupDev> groups;

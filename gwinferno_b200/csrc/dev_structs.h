@@ -1,5 +1,6 @@
 // Device-visible, trivially copyable mirrors of the plan (passed to kernels by value / pointer).
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <cstdlib>
 
@@ -70,6 +71,22 @@ PdlLauncher<KArgs...> make_pdl_launcher(void (*k)(KArgs...), dim3 g, dim3 b, siz
 namespace gwi {
 
 constexpr double SPEC_SHIFT_TOL = 300.0;  // p = e^(x - shift) within e^+-300 at the maximum: p and p^2 (N_eff sums) stay far from the fp64 limits
+
+// Power-law normaliser (distributions.py:111-116), shared by the prologue (SOP_POWERLAW_NORM, KOP_PLPEAK) and the stream
+// kernel (KOP_PLRATIO, per sample): lognorm = -log int_lo^hi x^(a1-1) dx and d lognorm / d a1, given log lo, L = log(hi/lo)
+// and inv_a1 = 1/a1 (0 at a1 = 0; the stream kernel takes it from the prologue instead of dividing per sample).
+// With z = a1 L the integral is lo^a1 L expm1(z)/z = lo^a1 expm1(z)/a1, so lognorm = -a1 log lo - log(expm1(z)/a1) (-log L at
+// z = 0) and the derivative is -log lo - L g(z), g(z) = 1/(1 - e^-z) - 1/z, i.e. 1/a1 - log hi - L/expm1(z).  No difference of
+// powers and no switch near a1 = 0 (alpha = -1).  The direct form of g loses ~eps/|z| to cancellation, so below |z| = 0.1 g is
+// its series (Bernoulli numbers; the first omitted term is < 3e-17 there).
+__device__ __forceinline__ void powerlaw_lognorm(double a1, double inv_a1, double loglo, double L, double& lognorm, double& dnorm) {
+  const double z = a1 * L;
+  const double em1 = expm1(z);
+  lognorm = -a1 * loglo - log(z != 0.0 ? em1 * inv_a1 : L);
+  const double z2 = z * z;
+  dnorm = fabs(z) < 0.1 ? -loglo - L * (0.5 + z * (1.0 / 12.0 + z2 * (-1.0 / 720.0 + z2 * (1.0 / 30240.0 - z2 * (1.0 / 1209600.0)))))
+                        : inv_a1 - (loglo + L) - L / em1;
+}
 
 struct DimDev {
   int32_t rows, row_off, slot, n_splines;

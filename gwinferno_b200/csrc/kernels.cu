@@ -95,28 +95,30 @@ __device__ double digamma_dev(double x) {
 __device__ __forceinline__ double norm_pdf(double x) { return exp(-0.5 * x * x) * 0.3989422804014327; }
 
 // log-normalisation of the truncated normal and the two ratios its gradient needs
-// (distributions.py:122-143): D = Phi(b) - Phi(a)
+// (distributions.py:122-143): D = Phi(b) - Phi(a), formed where it keeps its relative accuracy:
+//   - an interval narrow against the curvature of phi (half-width h, midpoint m): the series
+//     D = 2h phi(m) sum_k He_2k(m) h^2k / (2k+1)!  (He: Hermite polynomials; terms after h^6 are < 1e-17 there);
+//   - both bounds in one tail: the difference of erfc of that tail (the difference of two CDFs near 1 loses
+//     everything once the interval lies ~8 sigma out);
+//   - otherwise the difference of erf (no "1 +" to round away a small D).
 __device__ void truncnorm_consts(double mu, double sig, double lo, double hi, double& lognorm, double& dDmu_D, double& dDsig_D) {
   const double a = (lo - mu) / sig, b = (hi - mu) / sig;
-  const double D = 0.5 * (1.0 + erf(b * 0.7071067811865476)) - 0.5 * (1.0 + erf(a * 0.7071067811865476));
+  const double h = 0.5 * (hi - lo) / sig, m = (0.5 * (lo + hi) - mu) / sig;
+  const double r = 0.7071067811865476;
+  double D;
+  if (h * fmax(fabs(m), 1.0) < 0.01) {
+    const double m2 = m * m, h2 = h * h;
+    D = 2.0 * h * norm_pdf(m) * (1.0 + h2 * ((m2 - 1.0) * (1.0 / 6.0) + h2 * ((m2 * (m2 - 6.0) + 3.0) * (1.0 / 120.0) + h2 * (((m2 - 15.0) * m2 + 45.0) * m2 - 15.0) * (1.0 / 5040.0))));
+  } else if (a >= 0.0) {
+    D = 0.5 * (erfc(a * r) - erfc(b * r));
+  } else if (b <= 0.0) {
+    D = 0.5 * (erfc(-b * r) - erfc(-a * r));
+  } else {
+    D = 0.5 * (erf(b * r) - erf(a * r));
+  }
   lognorm = -log(sig) - 0.9189385332046727 - log(D);
   dDmu_D = (-norm_pdf(b) + norm_pdf(a)) / sig / D;
   dDsig_D = (-b * norm_pdf(b) + a * norm_pdf(a)) / sig / D;
-}
-
-// log[(1+a)/(hi^(1+a) - lo^(1+a))] and d/da (distributions.py:111-116)
-__device__ void powerlaw_lognorm(double alpha, double lo, double hi, double& lognorm, double& dnorm) {
-  const double a1 = 1.0 + alpha;
-  if (fabs(a1) < 1e-9) {
-    const double L = log(hi / lo);
-    lognorm = -log(L);
-    dnorm = -0.5 * (log(hi) + log(lo));  // limit of the derivative at alpha = -1
-    return;
-  }
-  const double ha = pow(hi, a1), la = pow(lo, a1);
-  const double den = ha - la;
-  lognorm = log(a1 / den);
-  dnorm = 1.0 / a1 - (ha * log(hi) - la * log(lo)) / den;
 }
 
 // Upper bound of the spline on polynomial piece J of dim D (convex-hull property: the bases are >= 0 and sum to <= 1):
@@ -364,10 +366,12 @@ __global__ void __launch_bounds__(256) prologue_kernel(const ModelDev* __restric
     } else if (K.kind == KOP_PLRATIO) {
       kc[0] = Lam[K.slot[0]];
       kc[1] = 1.0 + kc[0];
+      kc[2] = kc[1] != 0.0 ? 1.0 / kc[1] : 0.0;
     } else if (K.kind == KOP_PLPEAK) {
       const double alpha = Lam[K.slot[0]], mu = Lam[K.slot[1]], sig = Lam[K.slot[2]], lam = Lam[K.slot[3]];
       double ln, dn, lt, dmu, dsg;
-      powerlaw_lognorm(alpha, K.cst[0], K.cst[1], ln, dn);
+      const double a1 = 1.0 + alpha;
+      powerlaw_lognorm(a1, a1 != 0.0 ? 1.0 / a1 : 0.0, log(K.cst[0]), log(K.cst[1] / K.cst[0]), ln, dn);
       truncnorm_consts(mu, sig, K.cst[0], K.cst[1], lt, dmu, dsg);
       kc[0] = alpha; kc[1] = ln; kc[2] = mu; kc[3] = 0.5 / (sig * sig); kc[4] = lt; kc[5] = lam;
       kc[6] = dn; kc[7] = sig; kc[8] = dmu; kc[9] = dsg;
@@ -393,7 +397,8 @@ __global__ void __launch_bounds__(256) prologue_kernel(const ModelDev* __restric
       const SopDev& S = M.sops[q];
       if (S.kind == SOP_POWERLAW_NORM) {
         double ln, dn;
-        powerlaw_lognorm(Lam[S.slot0], S.cst0, S.cst1, ln, dn);
+        const double a1 = 1.0 + Lam[S.slot0];
+        powerlaw_lognorm(a1, a1 != 0.0 ? 1.0 / a1 : 0.0, log(S.cst0), log(S.cst1 / S.cst0), ln, dn);
         K += ln;
         M.Ksum[1 + S.slot0] += dn;
       } else if (S.kind == SOP_BETA_NORM) {
