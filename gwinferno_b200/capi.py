@@ -90,7 +90,7 @@ class gwi_model_desc(C.Structure):
         ("chunk_steps", C.c_int32),
         ("n_deep", C.c_int32),
         ("batch_hint", C.c_int32),
-        ("reserved_", C.c_int32),
+        ("keep_sample_index", C.c_int32),
     ]
 
 
@@ -148,6 +148,8 @@ SYMBOLS = [
     "gwi_sharded_push",
     "gwi_sharded_combine",
     "gwi_model_last_sites",
+    "gwi_sample_log_weights",
+    "gwi_draw_samples",
     "gwi_catalog_create",
     "gwi_catalog_destroy",
     "gwi_model_create",
@@ -229,6 +231,8 @@ def load_library(_allow_emulator=False):
     lib.gwi_model_last_sites.restype = C.c_int64
     lib.gwi_model_last_sites.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.c_int64]
     lib.gwi_model_set_exact_shift.argtypes = [C.c_void_p, C.c_int32]
+    lib.gwi_sample_log_weights.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.gwi_draw_samples.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     lib.gwi_model_set_timing.argtypes = [C.c_void_p, C.c_int32]
     lib.gwi_model_stream_times.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_int32]
     lib.gwi_debug_plan_build.argtypes = [C.c_void_p, C.POINTER(gwi_model_desc), C.c_int32, C.POINTER(C.c_void_p)]
@@ -374,7 +378,7 @@ def synth_injections_device(seed, first, count, device=0):
 class _Desc:
     """Keeps the ctypes structures and every NumPy array they point to alive."""
 
-    def __init__(self, spec, col_index, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0):
+    def __init__(self, spec, col_index, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0, keep_sample_index=False):
         self.keep = []
         nt = len(spec.terms)
         self.terms = (gwi_term * max(1, nt))()
@@ -433,7 +437,7 @@ class _Desc:
         d.chunk_steps = int(chunk_steps)
         d.n_deep = int(n_deep)
         d.batch_hint = int(batch_hint)
-        d.reserved_ = 0
+        d.keep_sample_index = int(bool(keep_sample_index))
         self.desc = d
 
 
@@ -554,9 +558,9 @@ class Catalog:
 class HostPlan:
     """Test hook: the static plan built on the host (no CUDA needed)."""
 
-    def __init__(self, catalog, spec, need_neff_grad=False, chunk_steps=0, n_deep=-1, n_workers=0, batch_hint=0):
+    def __init__(self, catalog, spec, need_neff_grad=False, chunk_steps=0, n_deep=-1, n_workers=0, batch_hint=0, keep_sample_index=False):
         lib = load_library()
-        self._d = _Desc(spec, catalog.col_index, need_neff_grad, chunk_steps, n_deep, batch_hint)
+        self._d = _Desc(spec, catalog.col_index, need_neff_grad, chunk_steps, n_deep, batch_hint, keep_sample_index)
         h = C.c_void_p()
         _check(lib.gwi_debug_plan_build(catalog.handle, C.byref(self._d.desc), int(n_workers), C.byref(h)))
         self.handle = h
@@ -586,14 +590,17 @@ class HostPlan:
 class Model:
     """gwi_model: the device-resident evaluation plan of one (catalog, model description)."""
 
-    def __init__(self, catalog, spec, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0):
+    def __init__(self, catalog, spec, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0, keep_sample_index=False):
+        """keep_sample_index=True: the model also keeps the catalog position of every stream position (4 bytes per padded
+        sample of device memory), which :meth:`sample_log_weights` and :meth:`draw_samples` need."""
         lib = load_library()
         self.catalog = catalog
+        self.keep_sample_index = bool(keep_sample_index)
         self.n_params = int(spec.n_params)
         self.n_events = catalog.n_events
         self.n_groups = len(spec.groups)
         self.need_neff_grad = bool(need_neff_grad)
-        self._d = _Desc(spec, catalog.col_index, need_neff_grad, chunk_steps, n_deep, batch_hint)
+        self._d = _Desc(spec, catalog.col_index, need_neff_grad, chunk_steps, n_deep, batch_hint, keep_sample_index)
         h = C.c_void_p()
         _check(lib.gwi_model_create(catalog.handle, C.byref(self._d.desc), C.byref(h)))
         self.handle = h
@@ -712,6 +719,46 @@ class Model:
             b.free()
         lam_d.free()
         return res
+
+    def _n_catalog(self):
+        return int(self.catalog.offsets[-1]) + int(self.catalog.n_inj)
+
+    def sample_log_weights(self, lam):
+        """gwi_sample_log_weights: log w of every catalog sample (``-inf`` where the weight is 0), PE samples in event order
+        followed by the injections, as one NumPy array.  Needs ``keep_sample_index=True``."""
+        lam = np.ascontiguousarray(lam, dtype=np.float64)
+        if lam.size != self.n_params:
+            raise ValueError(f"expected {self.n_params} hyper-parameters, got {lam.size}")
+        dev = self.catalog.device
+        lam_d, out_d = DeviceBuffer(self.n_params, dev), DeviceBuffer(self._n_catalog(), dev)
+        try:
+            lam_d.upload(lam)
+            _check(load_library().gwi_sample_log_weights(self.handle, C.c_void_p(lam_d.ptr), C.c_void_p(out_d.ptr), None))
+            synchronize()
+            return out_d.download()
+        finally:
+            lam_d.free()
+            out_d.free()
+
+    def draw_samples(self, lam, seed, draws_per_event, draws_inj):
+        """gwi_draw_samples: ``(pe[E, draws_per_event], inj[draws_inj])`` int64 local indices drawn with probability
+        proportional to the weight (-1 for an event / injection set without weight).  Needs ``keep_sample_index=True``."""
+        lam = np.ascontiguousarray(lam, dtype=np.float64)
+        if lam.size != self.n_params:
+            raise ValueError(f"expected {self.n_params} hyper-parameters, got {lam.size}")
+        E, dpe, dinj = self.n_events, int(draws_per_event), int(draws_inj)
+        n = E * dpe + dinj
+        dev = self.catalog.device
+        lam_d, out_d = DeviceBuffer(self.n_params, dev), DeviceBuffer(n, dev)  # (8-byte items: int64 read back as bits)
+        try:
+            lam_d.upload(lam)
+            _check(load_library().gwi_draw_samples(self.handle, C.c_void_p(lam_d.ptr), int(seed) & 0xFFFFFFFFFFFFFFFF, dpe, dinj, C.c_void_p(out_d.ptr), None))
+            synchronize()
+            out = out_d.download().view(np.int64)[:n]
+        finally:
+            lam_d.free()
+            out_d.free()
+        return out[: E * dpe].reshape(E, dpe).copy(), out[E * dpe :].copy()
 
     # -- device-pointer calls (multi-GPU plumbing) --------------------------------------------
     def partial(self, lam_ptr, record_ptr, stream=None):

@@ -39,6 +39,9 @@ void launch_combine(const ModelDev* Md, const double* recs, int R, const gwi_lik
 void launch_partial_tail(const ModelDev* Md, double* rec, int n_params, int tail, const gwi_like_opts& o, double* out, const CommDev& C, unsigned long long epoch, int nc,
                          cudaStream_t st);
 void launch_exchange(const ModelDev* Md, const double* rec_local, const CommDev& C, unsigned long long epoch, int mode, const gwi_like_opts& o, double* out, cudaStream_t st);
+void launch_sample_log_weights(const ModelDev* Md, int64_t n_padded, const uint32_t* index, double* out, int64_t n_cat, cudaStream_t st);
+void launch_draws(const DrawScratch& D, uint64_t seed, int E, int dpe, int dinj, int64_t* out, cudaStream_t st);
+void draw_tiles(const std::vector<int64_t>& seg_off, std::vector<int32_t>& tile_off, std::vector<int32_t>& tile_seg);
 
 }  // namespace gwi
 
@@ -58,9 +61,9 @@ static int build_plan_noexcept(const CatalogView& cat, const gwi_model_desc& des
   }
 }
 
-static int build_plan_device_noexcept(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_cols, double* secs) {
+static int build_plan_device_noexcept(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_cols, uint32_t** d_index, double* secs) {
   try {
-    return build_plan_device(cat, desc, sm_count, plan, d_cols, secs);
+    return build_plan_device(cat, desc, sm_count, plan, d_cols, d_index, secs);
   } catch (const std::bad_alloc&) {
     set_error("out of host memory building the plan");
     return GWI_ERR_ALLOC;
@@ -145,6 +148,9 @@ struct gwi_model {
   bool timing = false;
   std::vector<cudaEvent_t> ev0, ev1;
   int64_t n_timed = 0;
+  // gwi_model_desc.keep_sample_index: catalog position per padded stream position (device memory, in allocs)
+  uint32_t* sample_index = nullptr;
+  DrawScratch draw{};  // gwi_draw_samples: allocated on first use (in allocs)
 };
 
 static void phase_mark(gwi_model* m, int i, cudaStream_t st) {
@@ -264,6 +270,20 @@ int64_t gwi_debug_model_read(const gwi_model* m, int32_t what, void* dst, int64_
     }
     return n;
   }
+  if (what == 7) {
+    const int64_t n = m->sample_index ? m->plan.n_padded : 0;
+    if (dst && n > 0) {
+      if (cap < n) return GWI_ERR_INVALID;
+      std::vector<uint32_t> h((size_t)n);
+      if (cudaMemcpy(h.data(), m->sample_index, (size_t)n * 4, cudaMemcpyDeviceToHost) != cudaSuccess) {
+        set_error("cudaMemcpy of the sample index failed");
+        return GWI_ERR_CUDA;
+      }
+      int64_t* d = (int64_t*)dst;
+      for (int64_t i = 0; i < n; ++i) d[i] = h[i] == SAMPLE_INDEX_PAD ? -1 : (int64_t)h[i];
+    }
+    return n;
+  }
   return plan_read(m->plan, what, dst, cap);
 }
 
@@ -333,6 +353,11 @@ static int64_t plan_read(const Plan& p, int32_t what, void* dst, int64_t cap) {
           v.push_back(bits);
         }
       }
+      break;
+    case 7:  // catalog position per padded stream position, -1 = lane padding
+      if (p.keep_index)
+        for (uint32_t c : p.sample_index) v.push_back(c == SAMPLE_INDEX_PAD ? -1 : (int64_t)c);
+      if (p.n_padded == 0) v.clear();  // (the builder keeps one element for an empty plan)
       break;
     default:
       return GWI_ERR_INVALID;
@@ -512,9 +537,10 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
   if (cat->view.on_device) dev_build = true;
   const auto t_plan0 = std::chrono::steady_clock::now();
   uint64_t* d_cols_built = nullptr;
+  uint32_t* d_index_built = nullptr;
   int rc = GWI_OK;
   if (dev_build) {
-    rc = build_plan_device_noexcept(cat->view, *desc, prop.multiProcessorCount, m->plan, &d_cols_built, m->plan_seconds + 1);
+    rc = build_plan_device_noexcept(cat->view, *desc, prop.multiProcessorCount, m->plan, &d_cols_built, &d_index_built, m->plan_seconds + 1);
     if (rc == PLAN_DEVICE_FALLBACK) {
       if (cat->view.on_device) {
         set_error("model too large for the device plan builder's tables and the catalog columns are device-resident");
@@ -536,6 +562,8 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
   }
   m->plan_on_device = dev_build;
   if (d_cols_built) m->allocs.push_back(d_cols_built);
+  if (d_index_built) m->allocs.push_back(d_index_built);
+  m->sample_index = d_index_built;
   Plan& p = m->plan;
   ModelDev& H = m->host;
   const int P = p.n_params, NS = (int)p.dims.size(), nseg = (int)p.segments.size();
@@ -656,6 +684,10 @@ int gwi_model_create(gwi_catalog* cat, const gwi_model_desc* desc, gwi_model** o
   if (!d_cols) {
     UP(upload(m, p.columns.data(), p.columns.size(), &d_cols));
     std::vector<uint64_t>().swap(p.columns);  // host copy no longer needed
+  }
+  if (p.keep_index && !m->sample_index) {  // host builder
+    UP(upload(m, p.sample_index.data(), p.sample_index.size(), &m->sample_index));
+    std::vector<uint32_t>().swap(p.sample_index);
   }
   m->bytes_per_eval = (int64_t)p.n_columns * p.n_padded * 8;
   H.columns = d_cols;
@@ -803,6 +835,83 @@ static int run_eval(gwi_model* m, const double* lam_dev, int nc, cudaStream_t st
   // the last reduction level (one task per segment) is fused into finish_kernel
   launch_finish(m->dev, H.n_segments, H.rec_doubles, nc, st);
   phase_mark(m, 4, st);
+  CUDA_TRY(cudaGetLastError());
+  return GWI_OK;
+}
+
+// the per-sample log-weights into out_dev (catalog order): the prologue's tables and kernel constants on `st`, the grid
+// normalisers on the aux stream, joined before the pass.  No stream kernel, no reduction: the per-segment results, the
+// speculative shift and the captured graphs of the likelihood calls are untouched (the a-priori shift blocks of the prologue
+// are not launched either).
+static int sample_log_weights(gwi_model* m, const double* lam_dev, double* out_dev, cudaStream_t st) {
+  const ModelDev& H = m->host;
+  cudaEventRecord(m->ev_fork, st);
+  cudaStreamWaitEvent(m->aux_stream, m->ev_fork, 0);
+  launch_prologue_groups(m->dev, lam_dev, H.n_groups, m->max_grid, 1, m->aux_stream);
+  cudaEventRecord(m->ev_join, m->aux_stream);
+  launch_prologue_tables(m->dev, lam_dev, H.n_groups, H.n_segments, true, 1, st, 0);
+  cudaStreamWaitEvent(st, m->ev_join, 0);  // the pass reads logZ
+  launch_sample_log_weights(m->dev, H.n_padded, m->sample_index, out_dev, m->plan.n_samples_pe + m->plan.n_samples_inj, st);
+  CUDA_TRY(cudaGetLastError());
+  return GWI_OK;
+}
+
+static int check_sample_call(gwi_model* m, const double* lambda_dev, const void* out_dev) {
+  if (!m || !lambda_dev || !out_dev) {
+    set_error("null argument");
+    return GWI_ERR_INVALID;
+  }
+  if (!m->sample_index) {
+    set_error("per-sample weights and draws need a model created with keep_sample_index = 1");
+    return GWI_ERR_UNSUPPORTED;
+  }
+  CUDA_TRY(cudaSetDevice(m->device));
+  return GWI_OK;
+}
+
+int gwi_sample_log_weights(gwi_model* m, const double* lambda_dev, double* out_dev, void* stream) {
+  const int rc = check_sample_call(m, lambda_dev, out_dev);
+  if (rc != GWI_OK) return rc;
+  return sample_log_weights(m, lambda_dev, out_dev, (cudaStream_t)stream);
+}
+
+int gwi_draw_samples(gwi_model* m, const double* lambda_dev, uint64_t seed, int32_t draws_per_event, int32_t draws_inj, int64_t* out_dev, void* stream) {
+  if (draws_per_event < 0 || draws_inj < 0) {
+    set_error("negative number of draws");
+    return GWI_ERR_INVALID;
+  }
+  int rc = check_sample_call(m, lambda_dev, out_dev);
+  if (rc != GWI_OK) return rc;
+  const Plan& p = m->plan;
+  const int E = (int)p.segments.size() - 1;
+  DrawScratch& D = m->draw;
+  if (!D.logw) {
+    // segments in catalog order: the events (plan segments 1..E), then the injections (plan segment 0)
+    std::vector<int64_t> seg_off(E + 2, 0);
+    for (int i = 0; i < E; ++i) seg_off[i + 1] = seg_off[i] + p.segments[i + 1].n_total;
+    seg_off[E + 1] = seg_off[E] + p.segments[0].n_total;
+    std::vector<int32_t> tile_off, tile_seg;
+    draw_tiles(seg_off, tile_off, tile_seg);
+    DrawScratch N{};
+    N.n_seg = E + 1;
+    N.n_tiles = (int32_t)tile_seg.size();
+    N.n_cat = seg_off[E + 1];
+    int64_t* d_off;
+    int32_t *d_toff, *d_tseg;
+    if ((rc = upload(m, seg_off.data(), seg_off.size(), &d_off)) != GWI_OK || (rc = upload(m, tile_off.data(), tile_off.size(), &d_toff)) != GWI_OK ||
+        (rc = upload(m, tile_seg.data(), tile_seg.size(), &d_tseg)) != GWI_OK || (rc = upload<double>(m, nullptr, (size_t)N.n_cat, &N.logw)) != GWI_OK ||
+        (rc = upload<double>(m, nullptr, (size_t)N.n_tiles, &N.tile_max)) != GWI_OK || (rc = upload<double>(m, nullptr, (size_t)N.n_tiles, &N.tile_cum)) != GWI_OK ||
+        (rc = upload<double>(m, nullptr, (size_t)N.n_seg, &N.seg_max)) != GWI_OK)
+      return rc;  // (what was allocated stays in m->allocs until gwi_model_destroy)
+    N.seg_off = d_off;
+    N.tile_off = d_toff;
+    N.tile_seg = d_tseg;
+    D = N;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = sample_log_weights(m, lambda_dev, D.logw, st);
+  if (rc != GWI_OK) return rc;
+  launch_draws(D, seed, E, draws_per_event, draws_inj, out_dev, st);
   CUDA_TRY(cudaGetLastError());
   return GWI_OK;
 }

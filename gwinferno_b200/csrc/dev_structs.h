@@ -169,6 +169,22 @@ struct ModelDev {
   int32_t* tail_counter;  // arrival counter of partial_tail_kernel (zero between evaluations)
 };
 
+// posterior-predictive draws (sample_draw.cuh) over the catalog-order log-weights: segment s = event s (s < E) or the injection
+// set (s = E) covers catalog positions [seg_off[s], seg_off[s+1]) and is cut into tiles of DRAW_TILE samples that never
+// straddle segments (tiles [tile_off[s], tile_off[s+1]) of segment s).  Allocated on the first draw, owned by the model.
+constexpr int DRAW_TILE = 256;
+struct DrawScratch {
+  double* logw = nullptr;       // [n_cat] log-weights, catalog order
+  double* tile_max = nullptr;   // [n_tiles]
+  double* tile_cum = nullptr;   // [n_tiles] inclusive prefix over the segment's tiles of sum exp(x - seg_max)
+  double* seg_max = nullptr;    // [n_seg]
+  const int64_t* seg_off = nullptr;   // [n_seg + 1]
+  const int32_t* tile_off = nullptr;  // [n_seg + 1]
+  const int32_t* tile_seg = nullptr;  // [n_tiles]
+  int32_t n_seg = 0, n_tiles = 0;
+  int64_t n_cat = 0;
+};
+
 // multi-GPU exchange (exchange_kernel): the exchange buffers of every rank as seen from this rank (peer
 // memory), passed to the kernel by value
 constexpr int MAX_RANKS = 16;

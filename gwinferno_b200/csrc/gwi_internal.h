@@ -27,6 +27,7 @@ constexpr int MAX_GSLOTS = 32;      // gradient slots of the non-spline operatio
 constexpr int MAX_SOPS = 16;        // scalar (sample-independent) normaliser operations
 constexpr int KC_STRIDE = 12;       // doubles of per-eval constants per kop
 constexpr int LANES = 32;
+constexpr uint32_t SAMPLE_INDEX_PAD = 0xFFFFFFFFu;  // Plan::sample_index of lane padding
 constexpr int UNROLL = 2;           // samples per lane per load (16-byte vector loads)
 // copies of the deep accumulators per warp: lanes l and l+16 share a slot (two update phases, half the
 // shared memory of fully lane-private copies)
@@ -141,6 +142,10 @@ struct Plan {
   int col_static = 0;
   int64_t n_padded = 0;
   std::vector<uint64_t> columns;  // [n_padded/64][n_columns][64]: blocks of one warp iteration
+  // gwi_model_desc.keep_sample_index: catalog position of the sample at every padded position (PE samples in event order,
+  // then the injections), SAMPLE_INDEX_PAD for lane padding.  Host builder only (the device builder writes device memory).
+  bool keep_index = false;
+  std::vector<uint32_t> sample_index;
   std::vector<Chunk> chunks;
   std::vector<int32_t> slice_begin;  // slice i = chunks [slice_begin[i], slice_begin[i+1]); warp = i % W
   std::vector<Segment> segments;  // segment 0 = injections, 1..E = events

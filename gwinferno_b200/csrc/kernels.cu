@@ -984,3 +984,6 @@ void launch_combine(const ModelDev* Md, const double* recs, int R, const gwi_lik
 }
 
 }  // namespace gwi
+
+// per-sample log-weights and posterior-predictive draws (gwi_sample_log_weights / gwi_draw_samples)
+#include "sample_draw.cuh"

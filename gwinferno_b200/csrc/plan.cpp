@@ -237,6 +237,7 @@ int plan_classify(int n_cat_columns, const gwi_model_desc& desc, Plan& plan, Pla
     return GWI_ERR_INVALID;
   }
   plan = Plan();
+  plan.keep_index = desc.keep_sample_index != 0;
   plan.n_params = desc.n_params;
   plan.n_terms = desc.n_terms;
   plan.g2 = desc.need_neff_grad != 0;
@@ -1044,6 +1045,7 @@ int plan_fill_host(const CatalogView& cat, const PlanInputs& in, const std::vect
   // ---- pass 2: fill the stream columns ------------------------------------------------------
   try {
     plan.columns.assign((size_t)plan.n_columns * (size_t)std::max<int64_t>(1, plan.n_padded), 0ull);
+    if (plan.keep_index) plan.sample_index.assign((size_t)std::max<int64_t>(1, plan.n_padded), SAMPLE_INDEX_PAD);
   } catch (const std::bad_alloc&) {
     set_error("out of host memory building the plan");
     return GWI_ERR_ALLOC;
@@ -1079,6 +1081,8 @@ int plan_fill_host(const CatalogView& cat, const PlanInputs& in, const std::vect
         const std::vector<uint32_t>& ord = order[s];
         const int64_t r0 = chunk_r0[c];  // first sorted rank of this chunk
         const int64_t n_c = chunk_nc[c];
+        // catalog position = the row in the PE columns (event order), or n_samples_pe + the row in the injection columns
+        const uint32_t cat_base = s == 0 ? (uint32_t)plan.n_samples_pe : 0u;
         for (int cc : used_cols) {
           std::vector<double>& g = gathered[cc];
           if ((int64_t)g.size() < n_c) g.resize(n_c);
@@ -1105,6 +1109,7 @@ int plan_fill_host(const CatalogView& cat, const PlanInputs& in, const std::vect
             const int64_t p = sub + (int64_t)(k / UNROLL) * (LANES * UNROLL) + lane * UNROLL + (k % UNROLL);
             if (r < n_c) {
               const int64_t j = r;  // row of the chunk-local sorted copy
+              if (plan.keep_index) plan.sample_index[p] = cat_base + ord[r0 + r];
               for (int d = 0; d < NS; ++d) {
                 int J = 0;
                 double u = 0.0;

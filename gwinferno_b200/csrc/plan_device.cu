@@ -156,7 +156,7 @@ __global__ void __launch_bounds__(256) pd_rate_kernel(const uint64_t* __restrict
 // sub-chunk of main warp w is [first + w steps 32, ...), lane l owns the sorted run [l steps, (l+1) steps) of that
 // sub-chunk, and step k of lane l sits at (k/UNROLL)(32 UNROLL) + l UNROLL + k%UNROLL
 __global__ void __launch_bounds__(256) pd_fill_kernel(const __grid_constant__ PdParams A, const PdChunk* __restrict__ chunks, int n_chunks, const uint32_t* __restrict__ idx, int64_t n_padded,
-                                                      int n_columns, uint64_t* __restrict__ columns, PdChunkStat* __restrict__ stats) {
+                                                      int n_columns, uint64_t* __restrict__ columns, PdChunkStat* __restrict__ stats, uint32_t* __restrict__ sample_index) {
   const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= n_padded) return;  // n_padded is a multiple of 64: whole warps leave
   int lo = 0, hi = n_chunks - 1;
@@ -177,6 +177,7 @@ __global__ void __launch_bounds__(256) pd_fill_kernel(const __grid_constant__ Pd
   // lane padding: a copy of the chunk's last valid sample (every term evaluates to finite values and no piece index
   // changes) with static log-weight -inf => weight 0
   const int64_t j = (int64_t)idx[C.src0 + (valid ? r : C.n_c - 1)];
+  if (sample_index) sample_index[p] = valid ? (uint32_t)j : SAMPLE_INDEX_PAD;  // j: the catalog position (PE samples, then injections)
   int64_t jj;
   const double* const* cols = pd_cols(A, j, jj);
   const size_t base = ((size_t)(p >> 6) * (size_t)n_columns) * 64 + (size_t)(p & 63);
@@ -348,8 +349,10 @@ double seconds_since(std::chrono::steady_clock::time_point& t0) {
 // Returns GWI_OK, an error, or PLAN_DEVICE_FALLBACK (the model does not fit this path's fixed-size tables: the caller uses the
 // host builder if the catalog is on the host).  On success *d_columns_out is the plan's device array (cudaMalloc'd; the
 // caller owns it) and plan.columns stays empty.  stats_seconds[4] = raw-column upload, keys + sort + bounds, host geometry, fill.
-int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_columns_out, double* stats_seconds) {
+int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_columns_out, uint32_t** d_index_out,
+                      double* stats_seconds) {
   *d_columns_out = nullptr;
+  *d_index_out = nullptr;
   const bool timing = std::getenv("GWI_PLAN_TIMING") != nullptr;
   auto t0 = std::chrono::steady_clock::now();
   double secs[4] = {0, 0, 0, 0};
@@ -579,6 +582,13 @@ int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm
     d_columns = (uint64_t*)p;
     buf.ptrs.push_back(p);
   }
+  uint32_t* d_index = nullptr;
+  if (plan.keep_index) {
+    if (!buf.alloc(&d_index, (size_t)std::max<int64_t>(1, plan.n_padded))) {
+      set_error("device plan build: out of device memory for the sample index");
+      return GWI_ERR_ALLOC;
+    }
+  }
   std::vector<PdChunkStat> cstat(n_chunks);
   if (n_chunks > 0) {
     std::vector<PdChunk> pc(n_chunks);
@@ -599,7 +609,7 @@ int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm
     PD_ALLOC(d_stat, n_chunks);
     PD_CUDA(cudaMemcpy(d_pc, pc.data(), sizeof(PdChunk) * n_chunks, cudaMemcpyHostToDevice));
     PD_CUDA(cudaMemcpy(d_stat, cstat.data(), sizeof(PdChunkStat) * n_chunks, cudaMemcpyHostToDevice));
-    GWI_LAUNCH(pd_fill_kernel, dim3((unsigned)((plan.n_padded + TB - 1) / TB)), dim3(TB), 0, 0)(A, d_pc, n_chunks, idx_sorted, plan.n_padded, plan.n_columns, d_columns, d_stat);
+    GWI_LAUNCH(pd_fill_kernel, dim3((unsigned)((plan.n_padded + TB - 1) / TB)), dim3(TB), 0, 0)(A, d_pc, n_chunks, idx_sorted, plan.n_padded, plan.n_columns, d_columns, d_stat, d_index);
     PD_CUDA(cudaGetLastError());
     PD_CUDA(cudaMemcpy(cstat.data(), d_stat, sizeof(PdChunkStat) * n_chunks, cudaMemcpyDeviceToHost));
   }
@@ -617,6 +627,10 @@ int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm
   plan_tree(plan);
   buf.release(d_columns);
   *d_columns_out = d_columns;
+  if (d_index) {
+    buf.release(d_index);
+    *d_index_out = d_index;
+  }
   if (stats_seconds)
     for (int i = 0; i < 4; ++i) stats_seconds[i] = secs[i];
   if (timing)

@@ -229,8 +229,10 @@ int plan_geometry(const gwi_model_desc& desc, int sm_count, const PlanInputs& in
 void plan_tree(Plan& plan);
 int plan_begin_segments(const CatalogView& cat, Plan& plan);
 CosmoView cosmo_view_host();
-// plan_device.cu: the order and fill stages as kernels on the catalog's GPU; *d_columns_out = the plan's device array
+// plan_device.cu: the order and fill stages as kernels on the catalog's GPU; *d_columns_out = the plan's device array,
+// *d_index_out = its sample index (desc.keep_sample_index; nullptr otherwise)
 constexpr int PLAN_DEVICE_FALLBACK = 1;  // the model exceeds the device builder's fixed tables: use the host builder
-int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_columns_out, double* stats_seconds);
+int build_plan_device(const CatalogView& cat, const gwi_model_desc& desc, int sm_count, Plan& plan, uint64_t** d_columns_out, uint32_t** d_index_out,
+                      double* stats_seconds);
 
 }  // namespace gwi

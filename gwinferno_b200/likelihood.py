@@ -30,14 +30,18 @@ _BUILDS = collections.Counter()  # (term kinds, sharing pattern) -> plans built;
 class PopulationLikelihood:
     """Device-resident plan for one (catalog, population model) pair; evaluate for many Lambda."""
 
-    def __init__(self, lowered, total_inj, device=0, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0, catalog_on_device=False):
+    def __init__(self, lowered, total_inj, device=0, need_neff_grad=False, chunk_steps=0, n_deep=-1, batch_hint=0, catalog_on_device=False,
+                 keep_sample_index=False):
+        """keep_sample_index=True: the device plan also records each sample's catalog position (4 bytes per sample), which
+        :meth:`sample_log_weights` and :meth:`posterior_predictive` need."""
         self.lowered = lowered
         self.spec = lowered.spec
         self.n_params = lowered.spec.n_params
         # catalog_on_device=True: the sample columns are placed in device memory first and the plan is built from there
         # (capi.Catalog(on_device=True)): the setting of a caller whose arrays already live on the GPU
         self.catalog = capi.Catalog(lowered.pe_cols, lowered.inj_cols, total_inj, device=device, on_device=catalog_on_device)
-        self.model = capi.Model(self.catalog, lowered.spec, need_neff_grad=need_neff_grad, chunk_steps=chunk_steps, n_deep=n_deep, batch_hint=batch_hint)
+        self.model = capi.Model(self.catalog, lowered.spec, need_neff_grad=need_neff_grad, chunk_steps=chunk_steps, n_deep=n_deep, batch_hint=batch_hint,
+                                keep_sample_index=keep_sample_index)
         self.need_neff_grad = need_neff_grad
         self.n_events = self.catalog.n_events
 
@@ -68,6 +72,28 @@ class PopulationLikelihood:
     def info(self):
         return self.model.info()
 
+    def sample_log_weights(self, lam, host_log_norm=0.0):
+        """Per-sample population log-weights ``log p_pop(theta | Lambda) - log prior(theta)``, every normaliser included
+        (``-inf`` where the weight is 0): ``(pe, inj)`` with ``pe`` ``(E, S)`` (a list of per-event arrays for ragged
+        events) and ``inj`` ``(I,)``.  ``host_log_norm``: the host-side normaliser of the weights
+        (``lowering.host_log_norm(pe_weights, n_params)[0]``), subtracted here, so that ``logsumexp(pe[i]) - log S_i`` is
+        the ``logBFs`` site of event i and ``logsumexp(inj) - log total_inj`` the log detection efficiency.  Exponentiated
+        and normalised per event they are the population-reweighted event posteriors."""
+        x = self.model.sample_log_weights(lam) - float(host_log_norm)
+        off = self.catalog.offsets
+        pe = [x[off[i] : off[i + 1]] for i in range(self.n_events)]
+        if self.n_events and len({a.size for a in pe}) == 1:
+            pe = x[: off[-1]].reshape(self.n_events, -1)
+        return pe, x[off[-1] :]
+
+    def posterior_predictive(self, lam, seed=0, draws_per_event=1, draws_inj=None):
+        """Weighted draws (the reference's posterior-predictive resampling, analysis.py:321-355): ``(pe_idx[E,
+        draws_per_event], inj_idx[draws_inj])`` int64 sample indices inside each event / into the injection columns, drawn
+        with probability proportional to the weight; -1 where an event (or the injection set) has no weight.
+        ``draws_inj`` defaults to E.  Counter-based (Philox4x32-10 keyed by ``seed``): the same arguments give the same
+        draws, whatever the plan geometry."""
+        return self.model.draw_samples(lam, seed, draws_per_event, self.n_events if draws_inj is None else draws_inj)
+
 
 class LikelihoodResult:
     """What the reference's hierarchical_likelihood leaves in the NumPyro trace (analysis.py:260-319)."""
@@ -92,6 +118,7 @@ class LikelihoodResult:
         self._lowered = lowered
         self._pe_weights = pe_weights
         self.rate = None
+        self.ppc = None  # posterior_predictive_check=True: {"obs_index", "pred_index", "obs": {name: [E]}, "pred": {name: [E]}}
 
     def grad(self, param):
         """Gradient of log_l with respect to a parameter OBJECT that was passed to the model calls
@@ -135,9 +162,21 @@ def hierarchical_likelihood(
     """Drop-in for ``gwinferno.pipeline.analysis.hierarchical_likelihood`` (analysis.py:139-356)
     on lazy weights.  ``log=True`` takes lazy LOG-weights (``log_prob`` terms combined with ``+`` and
     ``- jnp.log(prior)``, analysis.py:401-421); the fused path always works in log space, so both forms
-    lower to the same device model.  The categorical sub-population branch (:246-254) and posterior-predictive
-    resampling (:321-355, with it ``param_names`` / ``pedata`` / ``injdata`` / ``m2min`` / ``m1min`` / ``mmax``)
-    are outside the fused hot path and raise NotImplementedError.  ``reconstruct_rate`` (:265-268): NumPyro
+    lower to the same device model.  The categorical sub-population branch (:246-254) is outside the fused path
+    and raises NotImplementedError.
+
+    ``posterior_predictive_check=True`` (:321-355) needs ``param_names``, ``pedata`` (dict name -> ``(E, S)`` array, or a
+    list of per-event arrays) and ``injdata`` (dict name -> ``(I,)`` array); without them it raises NotImplementedError.
+    It evaluates on a device plan that keeps each sample's catalog position (a separate cached engine) and draws, with
+    probability proportional to the population weight, one PE sample per event and E found injections on the GPU
+    (``PopulationLikelihood.posterior_predictive``, Philox4x32-10 keyed by ``rngkey``, 0 when None; not JAX's stream).
+    The drawn values are returned in ``res.ppc = {"obs_index", "pred_index", "obs": {name: [E]}, "pred": {name: [E]}}``
+    and as the sites ``{name}_obs_event_{i}`` / ``{name}_pred_event_{i}`` (NaN where an event has no weight); ``log_l``
+    and the gradient are those of the call without it.  The reference's source was not available when this was
+    written: these site names follow its description, not its code, and ``m1min`` / ``m2min`` / ``mmax``, whose role
+    there could not be checked, are accepted and unused.
+
+    ``reconstruct_rate`` (:265-268): NumPyro
     draws ``unscaled_rate ~ Gamma(Nobs)`` from the trace's key; here it is drawn from
     ``numpy.random.default_rng(rngkey)`` (``rngkey``: an int seed or ``None``) when a surveyed hypervolume is
     given, and returned -- as in the reference -- as the function's ``rate`` (``LikelihoodResult.rate``)."""
@@ -150,10 +189,11 @@ def hierarchical_likelihood(
         raise ValueError("log=True expects log-weights (built from log_prob with + / -), log=False expects weights (built with * and /)")
     if categorical or marginal_qs:
         raise NotImplementedError("the categorical sub-population branch is not part of the fused path")
-    if posterior_predictive_check:
-        raise NotImplementedError("posterior-predictive resampling (analysis.py:321-355) is not part of the fused path: draw from the per-sample weights on the host")
+    ppc = bool(posterior_predictive_check)
+    if ppc and (param_names is None or pedata is None or injdata is None):
+        raise NotImplementedError("posterior_predictive_check=True needs param_names, pedata and injdata (the sample values the draws are read from)")
     keys, pattern = lowering._structure(pe_weights, inj_weights)
-    cache_key = (keys, pattern, float(total_inj), bool(marginalize_selection), int(device))
+    cache_key = (keys, pattern, float(total_inj), bool(marginalize_selection), int(device), ppc)
     eng = _ENGINES.get(cache_key)
     if eng is None:
         shape_key = (tuple(k[0] if isinstance(k[0], str) else k[1] for k in keys), pattern)
@@ -161,7 +201,8 @@ def hierarchical_likelihood(
         if _BUILDS[shape_key] == 4:
             warnings.warn("hierarchical_likelihood built a new device plan for the same model shape 4 times: a model object or sample array is "
                           "re-created on every call (construct the models once, outside the sampled function)", RuntimeWarning, stacklevel=2)
-        eng = PopulationLikelihood.from_weights(pe_weights, inj_weights, total_inj, device=device, need_neff_grad=bool(marginalize_selection))
+        extra = dict(keep_sample_index=True) if ppc else {}
+        eng = PopulationLikelihood.from_weights(pe_weights, inj_weights, total_inj, device=device, need_neff_grad=bool(marginalize_selection), **extra)
         _ENGINES[cache_key] = eng
         while len(_ENGINES) > _MAX_ENGINES:
             _, old = _ENGINES.popitem(last=False)
@@ -187,7 +228,36 @@ def hierarchical_likelihood(
         unscaled = float(np.random.default_rng(rngkey).gamma(Nobs))
         res.sites["unscaled_rate"] = unscaled
         res.rate = res.sites["rate"] = unscaled / float(np.exp(head["log_mu"])) / total_vt
+    if ppc:
+        _posterior_predictive(res, eng, lam, rngkey, param_names, pedata, injdata)
     return res
+
+
+def _seed_of(rngkey):
+    """An integer seed from ``rngkey``: an int, None (0), or an array of key words (the last two, as JAX keys hold them)."""
+    if rngkey is None:
+        return 0
+    w = np.asarray(rngkey).ravel()
+    if w.size == 1:
+        return int(w[0]) & 0xFFFFFFFFFFFFFFFF
+    return ((int(w[-2]) & 0xFFFFFFFF) << 32) | (int(w[-1]) & 0xFFFFFFFF)
+
+
+def _posterior_predictive(res, eng, lam, rngkey, param_names, pedata, injdata):
+    """One PE sample per event ("obs") and E found injections ("pred") drawn by weight (analysis.py:321-355)."""
+    E = eng.n_events
+    pe_idx, inj_idx = eng.posterior_predictive(lam, seed=_seed_of(rngkey), draws_per_event=1, draws_inj=E)
+    obs_index = pe_idx[:, 0]
+    obs, pred = {}, {}
+    for name in param_names:
+        ev = pedata[name]
+        obs[name] = np.array([np.asarray(ev[i], dtype=np.float64)[obs_index[i]] if obs_index[i] >= 0 else np.nan for i in range(E)])
+        inj = np.asarray(injdata[name], dtype=np.float64)
+        pred[name] = np.where(inj_idx >= 0, inj[np.maximum(inj_idx, 0)], np.nan) if inj.size else np.full(inj_idx.shape, np.nan)
+        for i in range(E):
+            res.sites[f"{name}_obs_event_{i}"] = float(obs[name][i])
+            res.sites[f"{name}_pred_event_{i}"] = float(pred[name][i])
+    res.ppc = {"obs_index": obs_index, "pred_index": inj_idx, "obs": obs, "pred": pred}
 
 
 def apply_host_norm(log_l, grad, head, logZ, dlogZ, n_events, Nobs):

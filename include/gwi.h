@@ -143,7 +143,9 @@ typedef struct {
                              The machine is then filled by chains, so one chain's work is cut into 1/batch_hint as many,
                              batch_hint times longer slices (fewer record flushes, longer piece-sorted runs): 1.9x on the
                              1024-chain configuration.  Any chain count still works with any hint. */
-  int32_t reserved_;
+  int32_t keep_sample_index; /* 1: the model also keeps, per padded stream position, the catalog position of its sample
+                                (4 bytes per padded sample of device memory), which gwi_sample_log_weights and
+                                gwi_draw_samples need; 0: the plan exactly as without it */
 } gwi_model_desc;
 
 /* ---- catalog ------------------------------------------------------------------------------ */
@@ -305,6 +307,25 @@ int gwi_model_batch_hint(const gwi_model* m);
  * written (4 (E + 1)), or the number needed when dst == NULL, or a negative error. */
 int64_t gwi_model_last_sites(gwi_model* m, double* dst_host, int64_t cap_doubles);
 
+/* ---- per-sample weights and posterior-predictive draws (models created with keep_sample_index) ----------------
+ * Population-reweighted event posteriors and the posterior-predictive check of the reference (analysis.py:321-355,
+ * numpyro's random.choice(p = w / sum w) per event and over the found injections).  Neither call touches the state of the
+ * likelihood calls (speculative shift, captured graphs, the per-segment results of gwi_model_last_sites).
+ *
+ * log w of every catalog sample (log p_pop - log prior, every normaliser included; -inf where the weight is 0):
+ * out_dev [n_samples_pe + n_samples_inj] doubles, catalog order.  Asynchronous on `stream`.
+ * GWI_ERR_UNSUPPORTED unless the model was created with keep_sample_index. */
+int gwi_sample_log_weights(gwi_model* m, const double* lambda_dev, double* out_dev, void* stream);
+/* draws_per_event draws from each event's samples and draws_inj from the found injections, with probability
+ * proportional to the weight: out_dev [E * draws_per_event + draws_inj] int64 local indices (event i's draws first, at
+ * i * draws_per_event; an injection's local index is its index in the injection columns); -1 for a segment without weight.
+ * Draw k of segment s (s = i for event i, s = E for the injections) takes u = u01 of the first two words of
+ * Philox4x32-10 with counter (k, s, 0, 0) and key (seed_lo, seed_hi) and returns the first sample whose inclusive prefix
+ * sum of w / max w exceeds u times the segment total: deterministic, and independent of the plan geometry.
+ * Scratch (log-weights and tile sums, 8 bytes per catalog sample + a little) is allocated on first use and freed by
+ * gwi_model_destroy.  Asynchronous on `stream`. */
+int gwi_draw_samples(gwi_model* m, const double* lambda_dev, uint64_t seed, int32_t draws_per_event, int32_t draws_inj, int64_t* out_dev, void* stream);
+
 /* Log-sum-exp reference point.  By default spline-only models use an a-priori upper bound of the
  * per-sample log-weight per segment (single pass); if the bound is so loose for some Lambda that every
  * weight of a segment underflows, the asynchronous calls report GWI_LIKE_STATUS = 1 and
@@ -418,10 +439,13 @@ void gwi_debug_plan_destroy(gwi_plan* p);
  *       5 = non-spline op table [n_ops * 8] int64 {kind, column0, column1, slot0..slot3, bits of cst0}
  *       6 = per-segment statistics behind the a-priori shift [n_segments * 41] int64 {bits of max static weight,
  *           occupied pieces[8], bits of LIN feature min[16], max[16]}
+ *       7 = catalog position of the sample at every padded stream position [n_padded] int64, -1 for lane padding
+ *           (keep_sample_index models only; 0 items otherwise).  PE samples are numbered in event order by pe_offsets,
+ *           the injections follow them.
  * Returns the number of 8-byte items written (or needed when dst == NULL). */
 int64_t gwi_debug_plan_read(const gwi_plan* p, int32_t what, void* dst, int64_t cap_items);
-/* The same reader on a live model (what = 0, 2, 3, 4, 5 as above; what = 1 copies the plan's stream columns back
- * from device memory): lets the tests compare the device-built plan with the host-built one. */
+/* The same reader on a live model (what = 0, 2, 3, 4, 5 as above; what = 1 and 7 copy the plan's stream columns / sample
+ * index back from device memory): lets the tests compare the device-built plan with the host-built one. */
 int64_t gwi_debug_model_read(const gwi_model* m, int32_t what, void* dst, int64_t cap_items);
 
 #ifdef __cplusplus
